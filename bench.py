@@ -235,6 +235,37 @@ def forward_eval(model):
     return model.forward()
 
 
+DUMP_BYTES = 64 << 20
+DUMP_NAMES = {"a": "propagation", "b": "projection", "c": "topk_items", "c4096": "topk_items_batch4096"}
+
+
+def dump_outputs(dump_dir, outs):
+    """Write what each timed section returned to its caller as <dump_dir>/<name>.npy: `model.forward` -> propagation_<k>
+    (k-th returned tensor, user then item embeddings), the two modality projections -> projection_<k>, `full_sort_topk` of
+    all users -> topk_items, and of the 4096-user batches -> topk_items_batch4096 (the batches stacked).  Embeddings are
+    written as float32, item indices as float64 (exact).  When together they exceed 64 MiB, each array bigger than its share
+    keeps a fixed seeded sample of its rows, whose row numbers go to <name>.rows.npy."""
+    arrays = {}
+    for sec, out in outs.items():
+        if sec == "c4096":
+            arrays[DUMP_NAMES[sec]] = torch.cat(out)
+        elif torch.is_tensor(out):
+            arrays[DUMP_NAMES[sec]] = out
+        else:
+            arrays.update((f"{DUMP_NAMES[sec]}_{k}", t) for k, t in enumerate(out) if torch.is_tensor(t))
+    os.makedirs(dump_dir, exist_ok=True)
+    arrays = {k: t.detach().cpu().numpy() for k, t in arrays.items()}
+    arrays = {k: a.astype(np.float64 if a.dtype.kind in "iu" else np.float32) for k, a in arrays.items()}
+    share = DUMP_BYTES // (2 * len(arrays))                          # the other half bounds the row lists
+    sample = sum(a.nbytes for a in arrays.values()) > DUMP_BYTES
+    for name, a in arrays.items():
+        if sample and a.nbytes > share:
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], share // a[0].nbytes, replace=False))
+            np.save(os.path.join(dump_dir, name + ".rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(dump_dir, name + ".npy"), a)
+
+
 def torch_gpu_comparator(model, u_users, batches_dev, flush, reps=5):
     """The reference's own formulation on the same GPU with stock PyTorch kernels -- un-coalesced COO adjacency through
     `torch.sparse.mm` per layer + `stack().mean()` (`src/models/freedom.py:164-178`), `matmul` + in-place mask +
@@ -283,7 +314,7 @@ def torch_gpu_comparator(model, u_users, batches_dev, flush, reps=5):
 # ------------------------------------------------------------------------------------------------------
 # this repo's arm
 # ------------------------------------------------------------------------------------------------------
-def bench_model(wl, model_name, dev, args, flush, sampler=None, full=True):
+def bench_model(wl, model_name, dev, args, flush, sampler=None, full=True, dump_dir=None):
     """One model on one workload through the model-class API.  Device-timed sections (CUDA events, each section replayed
     from a CUDA graph -- kernels of 5-70 us are shorter than a Python call --, L2 flushed before every step):
         [A] `model.forward(...)`                       propagation, the plugin call of calculate_loss / full_sort_predict
@@ -356,6 +387,8 @@ def bench_model(wl, model_name, dev, args, flush, sampler=None, full=True):
                     times[name] += e0.elapsed_time(e1)
     ms = {k: v / steps for k, v in times.items()}
     launches = sum(n_launch[k] for k in n_launch if k != "c4096") * steps      # (the 4096-batch variant is an extra, not part of the step)
+    if dump_dir:                                                     # each replay rewrote the captured outputs: the last step's
+        dump_outputs(dump_dir, {name: graphs[name][1] for name, _ in secs})
 
     # ---- e2e through the same model calls, HOST buffers (pinned), copies inside the timed region.  [A]: the embedding
     # tables arrive from the host (a checkpoint / parameter-server push), forward, both outputs back.  [C]: the evaluation
@@ -464,6 +497,8 @@ def run_ours(args):
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     if world > 1 or args.sharded or args.workload == "xls":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the outputs of the single-GPU model-class path; the item-sharded driver has none")
         # the item-sharded driver; at world size 1 it is the weak-scaling baseline of the same per-GPU problem (no exchange)
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1"); os.environ.setdefault("MASTER_PORT", "29533")
         os.environ.setdefault("RANK", "0"); os.environ.setdefault("WORLD_SIZE", "1")
@@ -475,7 +510,7 @@ def run_ours(args):
     wl = Workload(args.workload, n_layers=3)
     flush = torch.empty(512 << 20, dtype=torch.uint8, device=dev)
     sampler = ClockSampler(local)
-    r = bench_model(wl, model_name, dev, args, flush, sampler, full=True)
+    r = bench_model(wl, model_name, dev, args, flush, sampler, full=True, dump_dir=args.dump_outputs)
     K = args.steps
     ms = r["ms"]
     msA, msB, msC = ms["a"], ms.get("b", 0.0), ms["c"]
@@ -657,7 +692,13 @@ def main():
     ap.add_argument("--sharded", action="store_true", help="run the item-sharded driver also at --gpus 1 (weak-scaling baseline)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the BM3/sports and MGCN/clothing lines in extra")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of this repo's CUDA path (--impl ours)")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

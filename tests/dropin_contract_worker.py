@@ -1,14 +1,17 @@
-"""Worker of tests/test_dropin_contract.py (own process: it imports the UNMODIFIED reference from /root/reference/src).
+"""Worker of tests/test_dropin_contract.py (own process: it replaces the kernels behind `mmrec_b200.ops` for its lifetime).
 
-INTEGRATION.md section 2 claims that `mmrec_b200.models.FREEDOM` is a drop-in under the reference's own `quick_start` /
-`Trainer` / dataloaders.  This proves the claim without a GPU: the reference's Config, RecDataset, TrainDataLoader,
-EvalDataLoader and Trainer are built exactly as `src/utils/quick_start.py:26-74` builds them, the model class is OURS, and the
-kernels behind `mmrec_b200.ops` are replaced by oracle-backed CPU stand-ins (test infrastructure: the product has no CPU
-path).  `Trainer.evaluate` (the reference's: full_sort_predict -> in-place mask -> torch.topk -> its own TopKEvaluator) must
-return the metrics recorded from the reference's own model, and one `calculate_loss` through `Trainer._train_epoch`'s call
-path must return the recorded loss."""
+INTEGRATION.md section 2 claims that `mmrec_b200.models.FREEDOM` is a drop-in for the reference's model under the
+reference's `quick_start` / `Trainer` / dataloaders.  This checks the claim without a GPU and without the reference: the
+package's restatement of that harness (Config, RecDataset, TrainDataLoader, EvalDataLoader, Trainer) is built exactly as
+`src/utils/quick_start.py:26-74` builds the reference's, the model class is OURS, and the kernels behind `mmrec_b200.ops` are
+replaced by oracle-backed CPU stand-ins (test infrastructure: the product has no CPU path).  What the reference's harness
+produced around the reference's own model -- its batches, losses and `Trainer.evaluate` metrics -- was recorded in
+tests/golden (make_golden.py); `Trainer.evaluate` on the dense route (full_sort_predict -> in-place mask -> torch.topk ->
+TopKEvaluator) must return those metrics, and one `calculate_loss` through `Trainer._train_epoch`'s call path must return
+the recorded loss."""
 import json
 import os
+import random
 import sys
 import tempfile
 
@@ -18,7 +21,8 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(HERE, "golden"))
+sys.path.insert(0, HERE)
+from conftest import load_golden  # noqa: E402
 
 
 class CpuCSR:
@@ -54,8 +58,10 @@ def install_cpu_ops():
     ops.project = lambda table, weight, bias=None, idx=None, l2_normalize=False: O.project(table, weight, bias, idx=idx, l2_normalize=l2_normalize)
     ops.score = lambda u, i, users=None: O.full_sort_scores(u, i, users if users is not None else torch.arange(u.shape[0]))
 
-    def mask_topk(scores, mask, k, item_offset=0):                    # graph._knn: selection of the kNN build
-        assert mask is None
+    def mask_topk(scores, mask, k, item_offset=0):                    # graph._knn, Trainer.evaluate's dense route
+        assert item_offset == 0
+        if mask is not None:
+            scores[mask[0], mask[1]] = -1e10                            # in place, as the reference's trainer.py:305-307
         return torch.topk(scores, k, dim=-1)
     ops.mask_topk = mask_topk
 
@@ -99,43 +105,43 @@ def install_cpu_ops():
     ops.propagate_layergcn = propagate_layergcn
 
 
-def main():
-    import ref_loader
+def harness(name, over):
+    """The tiny synthetic dataset on disk, then Config -> RecDataset -> loaders the way `src/utils/quick_start.py:26-74`
+    builds them, with the seed set as it sets it; the CPU stand-ins are installed last.  Returns (config, train, valid,
+    test, Trainer)."""
+    from mmrec_b200.common.trainer import Trainer
     from mmrec_b200.utils import synth
-    ref_loader.install()
-    tmp = tempfile.mkdtemp(prefix="mmrec_contract_")
-    data = ref_loader.run_dir(tmp)
+    from mmrec_b200.utils.configurator import Config
+    from mmrec_b200.utils.dataloader import EvalDataLoader, TrainDataLoader
+    from mmrec_b200.utils.dataset import RecDataset
+    from mmrec_b200.utils.utils import init_seed
+    data = os.path.join(tempfile.mkdtemp(prefix="mmrec_contract_"), "data")
     u, i, e, d, f = synth.SHAPES["tiny"]
     g = synth.make_graph(u, i, e, seed=0)
     v, t = synth.make_features(i, f, seed=1)
     synth.write_dataset(data, "tiny", g, v, t)
-    # --- the reference's own harness (src/utils/quick_start.py:26-74)
-    from utils.configurator import Config
-    from utils.dataset import RecDataset
-    from utils.dataloader import TrainDataLoader, EvalDataLoader
-    from utils.utils import init_seed
-    from common.trainer import Trainer
-    config = Config("FREEDOM", "tiny", {"gpu_id": 0, "use_gpu": False, "n_ui_layers": 3})
-    config["inter_file_name"] = "tiny.inter"
-    config["USER_ID_FIELD"], config["ITEM_ID_FIELD"] = "userID", "itemID"
-    config["vision_feature_file"], config["text_feature_file"] = "image_feat.npy", "text_feat.npy"
+    # the dense evaluation route (full_sort_predict -> mask -> top-k) of the reference's trainer: the stand-ins restate it
+    config = Config(name, "tiny", dict({"data_path": data + "/", "gpu_id": 0, "use_gpu": False, "use_fused_topk": False}, **over))
     for k in config["hyper_parameters"]:
         if isinstance(config[k], list):
             config[k] = config[k][0]
     dataset = RecDataset(config)
-    str(dataset)
     tr, va, te = dataset.split()
-    str(tr), str(va), str(te)
     train_data = TrainDataLoader(config, tr, batch_size=config["train_batch_size"], shuffle=True)
     valid_data = EvalDataLoader(config, va, additional_dataset=tr, batch_size=config["eval_batch_size"])
     test_data = EvalDataLoader(config, te, additional_dataset=tr, batch_size=config["eval_batch_size"])
     init_seed(config["seed"])
     train_data.pretrain_setup()
-    # --- OUR model class, the way utils.get_model would return it from src/models/freedom.py (INTEGRATION.md section 2)
     install_cpu_ops()
+    return config, train_data, valid_data, test_data, Trainer
+
+
+def main():
+    config, train_data, valid_data, test_data, Trainer = harness("FREEDOM", {"n_ui_layers": 3})
+    # --- OUR model class, the way utils.get_model would return it from src/models/freedom.py (INTEGRATION.md section 2)
     from mmrec_b200.models.freedom import FREEDOM
     model = FREEDOM(config, train_data).to(config["device"])
-    gold = np.load(os.path.join(HERE, "golden", "freedom_tiny.npz"), allow_pickle=True)
+    gold = load_golden("freedom_tiny.npz")
     sd = model.state_dict()
     init_identical = all(np.array_equal(sd[k[len("param0."):]].numpy(), gold[k]) for k in gold.files if k.startswith("param0."))
     trainer = Trainer(config, model)
@@ -159,41 +165,12 @@ def main():
 
 
 def main_mmgcn():
-    """The same for MMGCN: OUR class (no torch_geometric needed) under the reference's harness against
-    tests/golden/mmgcn_tiny.npz, the reference's own model code run under a PyG shim (tests/golden/ref_loader.py)."""
-    import ref_loader
-    from mmrec_b200.utils import synth
-    ref_loader.install()
-    tmp = tempfile.mkdtemp(prefix="mmrec_contract_")
-    data = ref_loader.run_dir(tmp)
-    u, i, e, d, f = synth.SHAPES["tiny"]
-    g = synth.make_graph(u, i, e, seed=0)
-    v, t = synth.make_features(i, f, seed=1)
-    synth.write_dataset(data, "tiny", g, v, t)
-    from utils.configurator import Config
-    from utils.dataset import RecDataset
-    from utils.dataloader import TrainDataLoader, EvalDataLoader
-    from utils.utils import init_seed
-    from common.trainer import Trainer
-    config = Config("MMGCN", "tiny", {"gpu_id": 0, "use_gpu": False, "eval_batch_size": 128, "train_batch_size": 512})
-    config["inter_file_name"] = "tiny.inter"
-    config["USER_ID_FIELD"], config["ITEM_ID_FIELD"] = "userID", "itemID"
-    config["vision_feature_file"], config["text_feature_file"] = "image_feat.npy", "text_feat.npy"
-    for k in config["hyper_parameters"]:
-        if isinstance(config[k], list):
-            config[k] = config[k][0]
-    dataset = RecDataset(config)
-    str(dataset)                                                    # (the reference computes inter_num / user_num in __str__)
-    tr, va, te = dataset.split()
-    str(tr), str(va), str(te)
-    train_data = TrainDataLoader(config, tr, batch_size=config["train_batch_size"], shuffle=True)
-    valid_data = EvalDataLoader(config, va, additional_dataset=tr, batch_size=config["eval_batch_size"])
-    init_seed(config["seed"])
-    train_data.pretrain_setup()
-    install_cpu_ops()
+    """The same for MMGCN: OUR class (no torch_geometric needed) against tests/golden/mmgcn_tiny.npz, the reference's own
+    model code run under a PyG shim (tests/golden/ref_loader.py)."""
+    config, train_data, valid_data, _, Trainer = harness("MMGCN", {"eval_batch_size": 128, "train_batch_size": 512})
     from mmrec_b200.models.mmgcn import MMGCN
     model = MMGCN(config, train_data).to(config["device"])
-    gold = np.load(os.path.join(HERE, "golden", "mmgcn_tiny.npz"), allow_pickle=True)
+    gold = load_golden("mmgcn_tiny.npz")
     sd = model.state_dict()
     init_identical = all(np.array_equal(sd[k[len("param0."):]].numpy(), gold[k]) for k in gold.files if k.startswith("param0.")) \
         and [k for k, _ in model.named_parameters()] == [str(x) for x in gold["param_order"]] \
@@ -221,45 +198,15 @@ def main_mmgcn():
 
 
 def main_model(name):
-    """BM3 / MGCN / LightGCN / LayerGCN: our class under the reference's harness against the golden file of the reference's
-    own class -- initial weights, `forward`, the loss on the recorded batch WITH the reference's RNG draws (BM3's always-on
-    dropout: same `torch.manual_seed(4321)` stream as tests/golden/make_golden.py), first-batch scores, `Trainer.evaluate`."""
-    import ref_loader
-    from mmrec_b200.utils import synth
-    ref_loader.install()
-    tmp = tempfile.mkdtemp(prefix="mmrec_contract_")
-    data = ref_loader.run_dir(tmp)
-    u, i, e, d, f = synth.SHAPES["tiny"]
-    g = synth.make_graph(u, i, e, seed=0)
-    v, t = synth.make_features(i, f, seed=1)
-    synth.write_dataset(data, "tiny", g, v, t)
-    from utils.configurator import Config
-    from utils.dataset import RecDataset
-    from utils.dataloader import TrainDataLoader, EvalDataLoader
-    from utils.utils import init_seed
-    from common.trainer import Trainer
+    """BM3 / MGCN / LightGCN / LayerGCN: our class against the golden file of the reference's own class -- initial
+    weights, `forward`, the loss on the recorded batch WITH the reference's RNG draws (BM3's always-on dropout: same
+    `torch.manual_seed(4321)` stream as tests/golden/make_golden.py), first-batch scores, `Trainer.evaluate`."""
     over = {"BM3": {}, "MGCN": {}, "LightGCN": {"n_layers": [3]}, "LayerGCN": {"dropout": [0.1]}}[name]
-    config = Config(name, "tiny", dict({"gpu_id": 0, "use_gpu": False, "eval_batch_size": 128, "train_batch_size": 512}, **over))
-    config["inter_file_name"] = "tiny.inter"
-    config["USER_ID_FIELD"], config["ITEM_ID_FIELD"] = "userID", "itemID"
-    config["vision_feature_file"], config["text_feature_file"] = "image_feat.npy", "text_feat.npy"
-    for k in config["hyper_parameters"]:
-        if isinstance(config[k], list):
-            config[k] = config[k][0]
-    dataset = RecDataset(config)
-    str(dataset)
-    tr, va, te = dataset.split()
-    str(tr), str(va), str(te)
-    train_data = TrainDataLoader(config, tr, batch_size=config["train_batch_size"], shuffle=True)
-    valid_data = EvalDataLoader(config, va, additional_dataset=tr, batch_size=config["eval_batch_size"])
-    test_data = EvalDataLoader(config, te, additional_dataset=tr, batch_size=config["eval_batch_size"])
-    init_seed(config["seed"])
-    train_data.pretrain_setup()
-    install_cpu_ops()
+    config, train_data, valid_data, test_data, Trainer = harness(name, dict({"eval_batch_size": 128, "train_batch_size": 512}, **over))
     import importlib
     cls = getattr(importlib.import_module("mmrec_b200.models." + name.lower()), name)
     model = cls(config, train_data).to(config["device"])
-    gold = np.load(os.path.join(HERE, "golden", name.lower() + "_tiny.npz"), allow_pickle=True)
+    gold = load_golden(name.lower() + "_tiny.npz")
     sd = model.state_dict()
     init_identical = all(np.array_equal(sd[k[len("param0."):]].numpy(), gold[k]) for k in gold.files if k.startswith("param0.")) \
         and [k for k, _ in model.named_parameters()] == [str(x) for x in gold["param_order"]]
@@ -305,23 +252,9 @@ def main_model(name):
 
 
 def main_traj(name):
-    """Two epochs of the reference's own training loop (`Trainer._train_epoch`, its Adam, its scheduler, its dataloader's
-    shuffling and negative sampling) driving OUR class, against the trajectory the reference's class produced
-    (tests/golden/traj_*_tiny.npz: every batch, every batch loss, per-epoch metrics)."""
-    import ref_loader
-    from mmrec_b200.utils import synth
-    ref_loader.install()
-    tmp = tempfile.mkdtemp(prefix="mmrec_contract_")
-    data = ref_loader.run_dir(tmp)
-    u, i, e, d, f = synth.SHAPES["tiny"]
-    g = synth.make_graph(u, i, e, seed=0)
-    v, t = synth.make_features(i, f, seed=1)
-    synth.write_dataset(data, "tiny", g, v, t)
-    from utils.configurator import Config
-    from utils.dataset import RecDataset
-    from utils.dataloader import TrainDataLoader, EvalDataLoader
-    from utils.utils import init_seed
-    from common.trainer import Trainer
+    """Two epochs of the reference's training loop as the package restates it (`Trainer._train_epoch`, torch's Adam, the
+    scheduler, the dataloader's shuffling and negative sampling) driving OUR class, against the trajectory the reference's
+    loop and class produced (tests/golden/traj_*_tiny.npz: every batch, every batch loss, per-epoch metrics)."""
     # key -> (model class, overrides of make_golden.py's dump_trajectory call, golden file)
     name, over, gfile = {"LightGCN": ("LightGCN", {"n_layers": [2], "reg_weight": [1e-4]}, "traj_lightgcn_tiny.npz"),
                          "FREEDOM": ("FREEDOM", {"dropout": [0.0], "reg_weight": [1e-3]}, "traj_freedom_tiny.npz"),
@@ -329,27 +262,11 @@ def main_traj(name):
                          "LayerGCN": ("LayerGCN", {"dropout": [0.1]}, "traj_layergcn_tiny.npz"),
                          "BM3": ("BM3", {}, "traj_bm3_tiny.npz"),
                          "MGCN": ("MGCN", {}, "traj_mgcn_tiny.npz")}[name]
-    config = Config(name, "tiny", dict({"gpu_id": 0, "use_gpu": False, "eval_batch_size": 128, "train_batch_size": 512}, **over))
-    config["inter_file_name"] = "tiny.inter"
-    config["USER_ID_FIELD"], config["ITEM_ID_FIELD"] = "userID", "itemID"
-    config["vision_feature_file"], config["text_feature_file"] = "image_feat.npy", "text_feat.npy"
-    for k in config["hyper_parameters"]:
-        if isinstance(config[k], list):
-            config[k] = config[k][0]
+    config, train_data, valid_data, test_data, Trainer = harness(name, dict({"eval_batch_size": 128, "train_batch_size": 512}, **over))
     config["epochs"] = 2
-    dataset = RecDataset(config)
-    str(dataset)
-    tr, va, te = dataset.split()
-    str(tr), str(va), str(te)
-    train_data = TrainDataLoader(config, tr, batch_size=config["train_batch_size"], shuffle=True)
-    valid_data = EvalDataLoader(config, va, additional_dataset=tr, batch_size=config["eval_batch_size"])
-    test_data = EvalDataLoader(config, te, additional_dataset=tr, batch_size=config["eval_batch_size"])
-    init_seed(config["seed"])
-    train_data.pretrain_setup()
-    install_cpu_ops()
     import importlib
     model = getattr(importlib.import_module("mmrec_b200.models." + name.lower()), name)(config, train_data).to(config["device"])
-    gold = np.load(os.path.join(os.environ.get("MMREC_TRAJ_DIR", os.path.join(HERE, "golden")), gfile), allow_pickle=True)
+    gold = load_golden(gfile, os.environ.get("MMREC_TRAJ_DIR"))
     trainer = Trainer(config, model)
     rec = {"batches": [], "losses": [], "valid": [], "test": []}
     orig = model.calculate_loss
@@ -360,9 +277,22 @@ def main_traj(name):
         rec["losses"].append(float(sum(l)) if isinstance(l, tuple) else float(l))
         return l
     model.calculate_loss = spy
+    # The package's loader draws negatives in numpy batches from a generator of its own, not one `random.sample` at a time
+    # (mmrec_b200/utils/dataloader.py), so where negatives are sampled the epochs replay the batches the reference's loader
+    # produced.  Without negatives (BM3) the loader must reproduce them itself.  The model's draws come from torch's
+    # generator, which neither loader touches, except LayerGCN's uniform pruning: it draws from Python's `random` after the
+    # reference's loader did, so each epoch starts from the state recorded there.
+    epochs = [train_data, train_data]
+    if config["use_neg_sampling"] is not False:
+        ends = np.cumsum(gold["batch_sizes"])
+        parts = [torch.from_numpy(np.ascontiguousarray(p)) for p in np.split(gold["batches"], ends[:-1], axis=1)]
+        first = int(gold["batches_per_epoch"][0])
+        epochs = [parts[:first], parts[first:]]
     for ep in range(2):
+        if "py_random_state" in gold:
+            random.setstate((3, tuple(int(x) for x in gold["py_random_state"][ep]), None))
         model.pre_epoch_processing()
-        trainer._train_epoch(train_data, ep)
+        trainer._train_epoch(epochs[ep], ep)
         trainer.lr_scheduler.step()
         rec["valid"].append(list(trainer.evaluate(valid_data).values()))
         rec["test"].append(list(trainer.evaluate(test_data).values()))

@@ -27,8 +27,10 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, HERE)
+sys.path.insert(0, os.path.dirname(HERE))
 
 import ref_loader  # noqa: E402
+from conftest import save_golden  # noqa: E402
 from mmrec_b200.utils import synth  # noqa: E402
 
 DATASET = "tiny"
@@ -165,7 +167,7 @@ def dump_model(model_name, overrides, out):
     # 2-epoch trajectory with recorded batches (device-RNG-free models only are replayable on GPU)
     if model_name in ("LightGCN", "FREEDOM0"):
         pass
-    np.savez_compressed(out, **g)
+    save_golden(out, g)
     print(f"{model_name}: wrote {out} ({os.path.getsize(out)/1024:.0f} KiB), valid={dict(zip(g['metric_names'][:4], g['metric_values'][:4]))}")
     return config, train_data, valid_data, test_data, model
 
@@ -215,12 +217,15 @@ def dump_mmgcn(overrides, out):
     res = Trainer(config, model).evaluate(valid_data)
     g["metric_names"] = np.array(list(res.keys()))
     g["metric_values"] = np.array([res[k] for k in res], dtype=np.float64)
-    np.savez_compressed(out, **g)
+    save_golden(out, g)
     print(f"MMGCN: wrote {out} ({os.path.getsize(out)/1024:.0f} KiB), loss {float(g['loss'][0]):.6f}")
 
 
-def dump_trajectory(model_name, overrides, out, epochs=2, slim=False):
-    """Train with the reference's own Trainer; record every batch, every batch loss, per-epoch metrics."""
+def dump_trajectory(model_name, overrides, out, epochs=2, slim=False, py_random=False):
+    """Train with the reference's own Trainer; record every batch, every batch loss, per-epoch metrics.  `py_random` also
+    records the state of Python's `random` at the start of each epoch: the reference's loader draws its negatives from it,
+    and LayerGCN's uniform pruning (`layergcn.py:56-58`) draws from it after them."""
+    import random
     from common.trainer import Trainer
     config, train_data, valid_data, test_data, model = build(model_name, overrides)
     config["epochs"] = epochs
@@ -237,8 +242,11 @@ def dump_trajectory(model_name, overrides, out, epochs=2, slim=False):
     model.calculate_loss = spy
     for k, p in model.state_dict().items():
         rec["param0." + k] = p.detach().numpy().copy()
-    batch_epoch = []
+    batch_epoch, py_states = [], []
     for ep in range(epochs):
+        state = random.getstate()
+        assert state[0] == 3 and state[2] is None
+        py_states.append(state[1])
         model.pre_epoch_processing()
         n0 = len(rec["batches"])
         trainer._train_epoch(train_data, ep)
@@ -258,7 +266,9 @@ def dump_trajectory(model_name, overrides, out, epochs=2, slim=False):
         if p.numel() <= 300 * 64 and not slim:
             g["paramT." + k] = p.detach().numpy().copy()
     g["learning_rate"] = np.float64(config["learning_rate"])
-    np.savez_compressed(out, **g)
+    if py_random:
+        g["py_random_state"] = np.array(py_states, dtype=np.int64)
+    save_golden(out, g)
     print(f"trajectory {model_name}: {len(rec['losses'])} batches, loss {rec['losses'][0]:.6f} -> {rec['losses'][-1]:.6f}, "
           f"valid recall@20 {g['valid'][:, list(g['metric_names']).index('recall@20')]}")
 
@@ -293,7 +303,8 @@ def main():
     for fcache in os.listdir(os.path.join(data_root, DATASET)):
         if fcache.endswith(".pt"):
             os.remove(os.path.join(data_root, DATASET, fcache))
-    dump_trajectory("LayerGCN", dict(common, dropout=[0.1]), os.path.join(HERE, "traj_layergcn_tiny.npz"), slim=True)
+    dump_trajectory("LayerGCN", dict(common, dropout=[0.1]), os.path.join(HERE, "traj_layergcn_tiny.npz"), slim=True,
+                    py_random=True)
     dump_trajectory("BM3", common, os.path.join(HERE, "traj_bm3_tiny.npz"), slim=True)
     dump_trajectory("MGCN", common, os.path.join(HERE, "traj_mgcn_tiny.npz"), slim=True)
 

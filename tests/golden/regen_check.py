@@ -1,5 +1,7 @@
-"""Worker of tests/test_dropin_contract.py::test_golden_files_are_what_the_reference_produces: re-run parts of make_golden.py
-against /root/reference into a scratch directory and compare with the committed files (build container only)."""
+"""Re-run parts of make_golden.py against a checkout of the reference (the one ref_loader.py imports) into a scratch
+directory and compare with the committed golden files: a model dump, the MMGCN dump under the PyG shim and a training
+trajectory -- every array bit for bit, recorded gradients to 1e-5 (CPU `index_put` backward is not run-to-run
+deterministic).  Prints one `REGEN {json}` line; needs the reference, so it is run by hand when a generator changes."""
 import json
 import os
 import sys
@@ -10,7 +12,9 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 sys.path.insert(0, HERE)
+sys.path.insert(0, os.path.dirname(HERE))
 import make_golden as M  # noqa: E402
+from conftest import load_golden  # noqa: E402
 import ref_loader  # noqa: E402
 from mmrec_b200.utils import synth  # noqa: E402
 
@@ -33,7 +37,7 @@ def main():
     M.dump_trajectory("BM3", common, os.path.join(out, "traj_bm3_tiny.npz"), slim=True)
     report = {}
     for name in ("lightgcn_tiny.npz", "mmgcn_tiny.npz", "traj_bm3_tiny.npz"):
-        a, b = np.load(os.path.join(out, name), allow_pickle=True), np.load(os.path.join(HERE, name), allow_pickle=True)
+        a, b = load_golden(name, out), load_golden(name, HERE)
         same_keys = sorted(a.files) == sorted(b.files)
         exact, worst = True, 0.0
         for k in b.files:
