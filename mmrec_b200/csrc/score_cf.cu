@@ -376,8 +376,12 @@ __device__ __forceinline__ float cf_scale_for(uint32_t m_bits) {
 }
 
 // One thread per (padded row, k block of 8): scale, round to fp16, store 16 bytes into the tile layout; the KP/8 threads
-// of a row are consecutive lanes and reduce the row's squared norm (and, for user rows, its largest magnitude) with
-// shuffles.  `scale_src` = the catalogue-wide largest magnitude (items), or NULL: per-row scale (users).
+// of a row are consecutive lanes and reduce, with shuffles, the row's largest magnitude (user rows) and then the squared
+// norm of the SCALED row.  `scale_src` = the catalogue-wide largest magnitude (items), or NULL: per-row scale (users).
+// The norm is taken after scaling so that it is valid for every finite row: the largest scaled element lies in
+// [2^14, 2^15), so a user row's sum of squares lies in [2^28, 2^37) whatever the magnitude of its elements (squares of the
+// unscaled elements underflow to 0 below ~1e-23 and overflow above ~2e18 at d = 64).  A catalogue row far below the
+// catalogue's largest element may underflow here, but such a row does not set the maximum norm.
 __device__ __forceinline__ void cf_pack_one(int64_t t, int64_t n_rows, const int64_t* __restrict__ idx, const float* __restrict__ E, int64_t ld,
                                             int d, int KP, const uint32_t* __restrict__ scale_src, uint4* __restrict__ out,
                                             float* __restrict__ row_norm, uint32_t* __restrict__ max_norm) {
@@ -393,27 +397,37 @@ __device__ __forceinline__ void cf_pack_one(int64_t t, int64_t n_rows, const int
         for (int e = 0; e < 8; ++e)
             if (kb * 8 + e < d) x[e] = __ldg(src + kb * 8 + e);
     }
-    float ss = 0.f;
-    uint32_t am = 0u;                                                 // largest |x| as a bit pattern (orders like the value; NaN above inf)
+    uint32_t am;
+    if (scale_src) {
+        am = __ldg(scale_src);
+    } else {
+        am = 0u;                                                      // largest |x| as a bit pattern (orders like the value; NaN above inf)
 #pragma unroll
-    for (int e = 0; e < 8; ++e) { ss = fmaf(x[e], x[e], ss); const uint32_t b = __float_as_uint(x[e]) & 0x7fffffffu; am = b > am ? b : am; }
-    for (int o = kblks / 2; o > 0; o >>= 1) {
-        ss += __shfl_xor_sync(0xffffffffu, ss, o);
-        const uint32_t a2 = __shfl_xor_sync(0xffffffffu, am, o);
-        am = a2 > am ? a2 : am;
+        for (int e = 0; e < 8; ++e) { const uint32_t b = __float_as_uint(x[e]) & 0x7fffffffu; am = b > am ? b : am; }
+        for (int o = kblks / 2; o > 0; o >>= 1) {
+            const uint32_t a2 = __shfl_xor_sync(0xffffffffu, am, o);
+            am = a2 > am ? a2 : am;
+        }
     }
-    const float sc = cf_scale_for(scale_src ? __ldg(scale_src) : am);
+    const float sc = cf_scale_for(am);
+    float ss = 0.f;
+#pragma unroll
+    for (int e = 0; e < 8; ++e) { x[e] *= sc; ss = fmaf(x[e], x[e], ss); }
+    for (int o = kblks / 2; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
     uint32_t w[4];
 #pragma unroll
     for (int e = 0; e < 4; ++e) {
-        const __half2 h = __floats2half2_rn(x[2 * e] * sc, x[2 * e + 1] * sc);
+        const __half2 h = __floats2half2_rn(x[2 * e], x[2 * e + 1]);
         w[e] = *reinterpret_cast<const uint32_t*>(&h);
     }
     const int64_t tile = row / CF_TILE;
     const int rr = (int)(row % CF_TILE);
     out[((tile * kblks + kb) * (CF_TILE / 8) + rr / 8) * 8 + (rr % 8)] = make_uint4(w[0], w[1], w[2], w[3]);
     if (kb == 0 && row < n_rows) {
-        const float nrm = sqrtf(ss) * sc * (1.0f + 1e-6f);            // norm of the scaled row (rounded up: the bound must hold)
+        // Rounded up so that the bound holds: ss sums at most 128 non-negative terms, and each term goes through at most
+        // 12 roundings (8 in the thread's fmaf chain, 4 in the shuffle tree at KP = 128), so ss is within 12 2^-24 = 7.2e-7
+        // of the exact sum; its square root is within 3.6e-7, plus 2^-24 for sqrtf and 2^-24 for the product: < 1e-6.
+        const float nrm = sqrtf(ss) * (1.0f + 1e-6f);
         if (row_norm) row_norm[row] = nrm;
         if (max_norm) atomicMax(max_norm, __float_as_uint(nrm));      // non-negative floats order like their bit patterns
     }

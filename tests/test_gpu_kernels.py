@@ -284,7 +284,10 @@ def _check_near_tie(idx, ref, ri, scale):
 
 def test_fused_topk_operand_scaling(dev):
     """The filter's fp16 operands are scaled by powers of two (per user row, per catalogue): tiny, huge and mixed
-    magnitudes must neither overflow nor lose the certificate (every row served by the filter, result = fp32 top-k)."""
+    magnitudes must neither overflow nor lose the certificate (every row served by the filter, result = fp32 top-k).
+    Random tables cannot exercise the filter's margin: the masked-item rows and the group granularity leave more slack
+    than fp16 rounding takes, so a wrong margin or a wrong row norm still passes here.  tests/test_gpu_score_cf.py holds
+    the adversarial catalogue, the exact power-of-two scale invariance and the fp64 acceptance rule that would catch it."""
     from mmrec_b200 import ops
     ops.set_score_path("fused")
     try:
